@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--dtype complex128] [--impl reference]
                     [--config m20|peps8x8|m10|m10s|m12] [--scaling weak|strong]
+                    [--dump-outputs DIR]
 
 Default workload (config.workload): the reference's own benchmark structure
 ``examples/benchmarks/sycamore_n53_m20_s0_e0_pABCDCDAB.json`` (381 tensors, 754
@@ -54,6 +55,7 @@ METRICS = {
 }
 UNIT = "TFLOP/s"
 SEED, SCALE = 0, 0.65
+DUMP_BYTES = 60 * 10**6  # --dump-outputs: arrays plus .npy headers stay under 64 MB
 
 
 # ---------------------------------------------------------------------------
@@ -203,7 +205,8 @@ class CpuSample:
 
     def run(self, i):
         t0 = time.perf_counter()
-        self.orc.run_contractions(self.ir, self.orc.slice_arrays(self.inputs, self.small.sliced, self.arrays, i))
+        self.last = self.orc.run_contractions(self.ir, self.orc.slice_arrays(self.inputs, self.small.sliced,
+                                                                              self.arrays, i))
         return time.perf_counter() - t0
 
 
@@ -275,7 +278,28 @@ def run_reference(args):
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     del ctl
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"out": s.last})
     print(json.dumps(line))
+
+
+def dump_outputs(dirname, outputs):
+    """``--dump-outputs``: each array of the timed path's last step as ``DIR/<name>.npy``, complex
+    values as (real, imag) pairs on a trailing axis in the precision they were computed in.  An
+    output larger than its share of ``DUMP_BYTES`` is replaced by a fixed seeded sample of its flattened
+    elements (ascending positions), so that two builds can be compared value for value."""
+    os.makedirs(dirname, exist_ok=True)
+    budget = DUMP_BYTES // max(1, len(outputs))
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        real = np.dtype(np.float64 if a.dtype in (np.complex128, np.float64) else np.float32)
+        per = real.itemsize * (2 if a.dtype.kind == "c" else 1)
+        if a.size * per > budget:
+            keep = np.random.default_rng(SEED).choice(a.size, budget // per, replace=False)
+            a = a.reshape(-1)[np.sort(keep)]
+        if a.dtype.kind == "c":
+            a = np.stack([a.real, a.imag], axis=-1)
+        np.save(os.path.join(dirname, f"{name}.npy"), a.astype(real))
 
 
 def dtype_tag(dtype):
@@ -511,6 +535,7 @@ def run_gpu(args):
 
     r = timed_run(ex, tensors, args, world, rank, dev, S)
     ms, launches, node_ms, clocks, out, barrier = (r[k] for k in ("ms", "launches", "node_ms", "clocks", "out", "barrier"))
+    dumped = {"out": out.cpu().numpy()}
     macs_ref, _macs_inv, elems_ref = ex.reference_work
     flops_slice = 8 * macs_ref
     total_slices = S * world * args.steps
@@ -552,6 +577,7 @@ def run_gpu(args):
         ex64 = cb.TreeExecutor(spec, dtype="complex64", device=local, fuse=not args.no_fuse)
         t64 = [t.to(torch.complex64) for t in tensors]
         r64 = timed_run(ex64, t64, args, world, rank, dev, S)
+        dumped["out_complex64"] = r64["out"].cpu().numpy()
         m64, _i64, _e64 = ex64.reference_work
         v64 = 8 * m64 * total_slices / (r64["ms"] * 1e-3) / 1e12
         if rank == 0:
@@ -668,6 +694,8 @@ def run_gpu(args):
         "gpu_library_baseline": gpu_lib,
         "cpu_baseline": cpu,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumped)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -688,6 +716,8 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the complex64 leg")
     ap.add_argument("--no-gpu-lib", action="store_true", help="skip the torch.tensordot GPU-library baseline")
     ap.add_argument("--no-fuse", action="store_true", help="execute the reference's node sequence one to one")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32/float64)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -351,13 +351,17 @@ def tensordot(a, b, axes=2):
 
 
 def run_contractions(
-    contractions, arrays, strip_exponent=False, check_zero=False
+    contractions, arrays, strip_exponent=False, check_zero=False,
+    implementation=None,
 ):
     """Contract ``arrays`` by walking the linear program ``contractions``.
 
     Returns the output array, or ``(mantissa, exponent)`` (base-10 exponent) if
-    ``strip_exponent``.
+    ``strip_exponent``.  ``implementation`` is an ``(einsum, tensordot)`` pair
+    that every node is dispatched to instead of this module's own, as the
+    reference's ``implementation=`` argument does (contract.py:752-776).
     """
+    einsum_, tensordot_ = implementation or (einsum, tensordot)
     live = dict(enumerate(arrays))
     exponent = 0.0 if strip_exponent else None
     out = None
@@ -365,19 +369,19 @@ def run_contractions(
         if r is None:
             if l is None:
                 # in-place preprocessing of input ``p``
-                live[p] = einsum_single(arg, live[p])
+                live[p] = einsum_(arg, live[p])
                 continue
             # single-input tree
-            out = einsum_single(arg, live[l])
+            out = einsum_(arg, live[l])
             return (out, 0.0) if strip_exponent else out
         x = live.pop(l)
         y = live.pop(r)
         if tdot:
-            out = tensordot(x, y, arg)
+            out = tensordot_(x, y, arg)
             if perm:
                 out = np.transpose(out, perm)
         else:
-            out = einsum(arg, x, y)
+            out = einsum_(arg, x, y)
         if exponent is not None:
             top = np.max(np.abs(out))
             if check_zero and float(top) == 0.0:

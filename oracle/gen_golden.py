@@ -481,8 +481,85 @@ def gen_sycamore():
     print("sycamore:", stats, tree.nslices, small.nslices, med.nslices)
 
 
+# --------------------------------------------------------------------------
+# 5. Freshly searched random trees (tests/test_tree_ir.py)
+# --------------------------------------------------------------------------
+
+
+def gen_random_trees():
+    """Greedy trees of random equations with random index orders, slicing and
+    removed indices: ``tree_record`` holds what ``TreeSpec.from_cotengra`` reads
+    and the reference's IR and slice keys it must reproduce."""
+    rng = random.Random(5)
+    recs = []
+    for trial in range(40):
+        c = ctg.utils.rand_equation(
+            n=rng.randint(4, 12), reg=rng.randint(2, 4), n_out=rng.randint(0, 3),
+            n_hyper_in=rng.randint(0, 2), n_hyper_out=rng.randint(0, 2),
+            d_min=1, d_max=4, seed=trial,
+        )
+        tree = ctg.array_contract_tree(
+            c.inputs, c.output, c.size_dict, optimize="greedy",
+            sort_contraction_indices=rng.choice([None, "root", "flops"]),
+        )
+        if tree.max_size() > 16 and rng.random() < 0.7:
+            tree.slice_(target_size=max(tree.max_size() // 4, 1))
+        rem = [ix for ix in tree.get_legs(tree.root)]
+        if rem and rng.random() < 0.5:
+            tree.remove_ind_(rng.choice(rem))
+        recs.append(tree_record(f"random_tree{trial}", tree, "complex128", seed=trial))
+    with open(os.path.join(GOLDEN_DIR, "random_trees.json"), "w") as f:
+        json.dump(recs, f)
+    print("random trees:", len(recs))
+
+
+# --------------------------------------------------------------------------
+# 6. The drop-in boundary (tests/test_dropin_reference.py)
+# --------------------------------------------------------------------------
+
+
+def gen_dropin():
+    """BASELINE config 1 (and its hyper-index variant) through the reference's
+    own entry points: ``ctg.einsum``, ``tree.contract`` (plain, stripped,
+    sliced), ``tree.contract_slice``, the keys its contractor cache used, and
+    ``total_flops`` of a sliced lattice tree."""
+    recs, vals = {}, {}
+    for hyper in (False, True):
+        kw = dict(n_out=2, n_hyper_in=1, n_hyper_out=1) if hyper else {}
+        con = ctg.utils.rand_equation(10, 3, d_min=4, d_max=4, seed=0, **kw)
+        shapes = [tuple(con.size_dict[ix] for ix in t) for t in con.inputs]
+        arrays = make_arrays(shapes, "complex128", seed=0)
+        eq = ctg.utils.inputs_output_to_eq(con.inputs, con.output)
+        tag = f"config1_hyper{int(hyper)}"
+        vals[f"{tag}_einsum"] = np.asarray(ctg.einsum(eq, *arrays))
+        tree = ctg.array_contract_tree(con.inputs, con.output, con.size_dict, optimize="greedy")
+        vals[f"{tag}_contract"] = np.asarray(tree.contract(arrays))
+        m, e = tree.contract(arrays, strip_exponent=True)
+        vals[f"{tag}_strip_m"], vals[f"{tag}_strip_e"] = np.asarray(m), np.asarray(e)
+        rec = tree_record(tag, tree, "complex128", seed=0)
+        rec["eq"] = eq
+        # (strip_exponent, key) of every contractor the calls above cached
+        rec["contractor_keys"] = [[bool(k[3]), jsonable(k)] for k in tree.contraction_cores]
+        recs[tag] = rec
+        if hyper:
+            tree.slice_(target_size=max(tree.max_size() // 8, 1))
+            vals["sliced_contract"] = np.asarray(tree.contract(arrays))
+            for i in (0, tree.nslices - 1):
+                vals[f"sliced_slice{i}"] = np.asarray(tree.contract_slice(arrays, i))
+            recs["sliced"] = tree_record("sliced", tree, "complex128", seed=0)
+    con = ctg.utils.lattice_equation([4, 4], d_min=3)
+    tree = ctg.array_contract_tree(con.inputs, con.output, con.size_dict, optimize="greedy")
+    tree.slice_(target_slices=9)
+    recs["lattice4x4"] = tree_record("lattice4x4", tree, "float64", seed=0,
+                                     extra={"total_flops_float64": int(tree.total_flops("float64"))})
+    with open(os.path.join(GOLDEN_DIR, "dropin.json"), "w") as f:
+        json.dump(recs, f)
+    np.savez_compressed(os.path.join(GOLDEN_DIR, "dropin_values.npz"), **vals)
+    print("dropin:", sorted(recs))
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["parsers", "equations", "trees", "sycamore"]
+    which = sys.argv[1:] or ["parsers", "equations", "trees", "sycamore", "random_trees", "dropin"]
     if "parsers" in which:
         gen_parsers()
     if "equations" in which:
@@ -491,3 +568,7 @@ if __name__ == "__main__":
         gen_trees()
     if "sycamore" in which:
         gen_sycamore()
+    if "random_trees" in which:
+        gen_random_trees()
+    if "dropin" in which:
+        gen_dropin()

@@ -3,6 +3,7 @@ tests: deterministic synthetic arrays and golden-file decoding."""
 
 import json
 import os
+from types import SimpleNamespace
 
 import numpy as np
 
@@ -50,6 +51,32 @@ def decode_ir(contractions):
 def decode_sliced(sliced):
     return [(ind, int(size), None if project is None else int(project))
             for ind, size, project in sliced]
+
+
+class RecordedTree:
+    """A ``cotengra.ContractionTree`` as ``oracle/gen_golden.tree_record`` stored it: the
+    attributes ``TreeSpec.from_cotengra`` reads (nodes are the record's SSA ids) and the
+    contractor cache ``cotengra_b200.install`` seeds."""
+
+    def __init__(self, rec):
+        self.inputs = [tuple(t) for t in rec["inputs"]]
+        self.output = tuple(rec["output"])
+        self.size_dict = dict(rec["size_dict"])
+        self.sliced_inds = {ix: SimpleNamespace(ind=ix, size=int(size), project=project)
+                            for ix, size, project in rec["sliced"]}
+        self._path = [tuple(p) for p in rec["path"]]
+        self._inds = {int(k): v for k, v in rec["inds"].items()}
+        self.contraction_cores = {}
+
+    def gen_leaves(self):
+        return iter(range(len(self.inputs)))
+
+    def traverse(self):
+        n = len(self.inputs)
+        return [(n + k, l, r) for k, (l, r) in enumerate(self._path)]
+
+    def get_inds(self, node):
+        return self._inds[node]
 
 
 def rel_err(x, ref):

@@ -1,5 +1,5 @@
-"""Host-side .qsim reader: gate set sanity (no GPU, no reference needed) and, in the
-build container, the structure of the reference's Sycamore circuit files."""
+"""Host-side .qsim reader: gate set sanity and the structure of the reference's Sycamore
+circuit files (copied under ``tests/golden/``)."""
 
 import os
 
@@ -7,6 +7,11 @@ import numpy as np
 import pytest
 
 from cotengra_b200.circuits import amplitude_network, gate_matrix, read_qsim
+from tests.helpers import GOLDEN_DIR, load_json
+
+
+def _qsim(m):
+    return os.path.join(GOLDEN_DIR, f"circuit_n53_m{m}_s0_e0_pABCDCDAB.qsim")
 
 
 def test_gates_are_unitary_and_square_roots():
@@ -28,9 +33,8 @@ def test_gates_are_unitary_and_square_roots():
         gate_matrix("cz", ())
 
 
-@pytest.mark.reference
 def test_sycamore_m10_network_structure():
-    path = "/root/reference/examples/circuit_n53_m10_s0_e0_pABCDCDAB.qsim"
+    path = _qsim(10)
     n, gates = read_qsim(path)
     assert n == 53 and len(gates) == 1658  # SURVEY.md Appendix C
     inputs, output, size_dict, arrays = amplitude_network(path)
@@ -83,7 +87,6 @@ def test_rank_simplify_small_circuit_keeps_the_amplitude(tmp_path):
     assert abs(a0 - a1) < 1e-12 * max(1.0, abs(a0))
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("m,tensors,indices", [(10, 164, 319), (20, 381, 754)])
 def test_rank_simplify_reaches_the_notebook_sizes(m, tensors, indices):
     """The reference notebooks contract networks simplified by quimb: m10 has 164 tensors / 319
@@ -91,7 +94,7 @@ def test_rank_simplify_reaches_the_notebook_sizes(m, tensors, indices):
     (`ex_benchmarking.ipynb` cell 4).  rank_simplify reproduces both counts from the .qsim files."""
     from cotengra_b200.circuits import rank_simplify
 
-    path = f"/root/reference/examples/circuit_n53_m{m}_s0_e0_pABCDCDAB.qsim"
+    path = _qsim(m)
     inputs, output, size_dict, arrays = amplitude_network(path)
     s_in, _o, s_sizes, s_arr = rank_simplify(inputs, output, size_dict, arrays)
     assert len(s_in) == tensors and len(s_sizes) == indices
@@ -102,10 +105,7 @@ def test_rank_simplify_reaches_the_notebook_sizes(m, tensors, indices):
             counts[ix] = counts.get(ix, 0) + 1
     assert set(counts.values()) == {2}
     if m == 20:
-        # same degree sequence as the reference's benchmark structure file
-        import json
-
-        with open("/root/reference/examples/benchmarks/sycamore_n53_m20_s0_e0_pABCDCDAB.json") as f:
-            ref = json.load(f)
-        ref_inputs = ref["inputs"] if isinstance(ref, dict) else ref[0]
+        # same degree sequence as the reference's benchmark structure file, whose network
+        # sycamore_m20.json carries
+        ref_inputs = next(r for r in load_json("sycamore_m20.json") if r["name"] == "sycamore_m20_appxB")["inputs"]
         assert sorted(len(t) for t in ref_inputs) == sorted(len(t) for t in s_in)

@@ -1,13 +1,10 @@
 """``TreeSpec`` regenerates the reference's contraction IR bit-exactly
 (integer/string work: pinned to golden records from the unmodified reference)."""
 
-import os
-import sys
-
 import pytest
 
 from cotengra_b200 import TreeSpec
-from tests.helpers import decode_ir, decode_sliced, load_json
+from tests.helpers import RecordedTree, decode_ir, decode_sliced, load_json
 
 TREES = load_json("trees.json") + load_json("sycamore_m20.json")
 
@@ -47,38 +44,15 @@ def test_ir_matches_reference(rec):
     assert again.contractions() == spec.contractions()
 
 
-@pytest.mark.reference
 def test_live_reference_random_trees():
-    """In the build container: compare against the live reference on freshly
-    generated trees (searches are unseeded, so these differ from the goldens)."""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    sys.path[:0] = [os.path.join(root, "oracle", "refshim"), "/root/reference"]
-    try:
-        import cotengra as ctg
-        refc = sys.modules["cotengra.contract"]
-        import random
-
-        rng = random.Random(5)
-        for trial in range(40):
-            c = ctg.utils.rand_equation(
-                n=rng.randint(4, 12), reg=rng.randint(2, 4), n_out=rng.randint(0, 3),
-                n_hyper_in=rng.randint(0, 2), n_hyper_out=rng.randint(0, 2),
-                d_min=1, d_max=4, seed=trial,
-            )
-            tree = ctg.array_contract_tree(
-                c.inputs, c.output, c.size_dict, optimize="greedy",
-                sort_contraction_indices=rng.choice([None, "root", "flops"]),
-            )
-            if tree.max_size() > 16 and rng.random() < 0.7:
-                tree.slice_(target_size=max(tree.max_size() // 4, 1))
-            rem = [ix for ix in tree.get_legs(tree.root)]
-            if rem and rng.random() < 0.5:
-                tree.remove_ind_(rng.choice(rem))
-            spec = TreeSpec.from_cotengra(tree)
-            want_pre, want = _split(tuple(refc.extract_contractions(tree)))
-            got_pre, got = _split(spec.contractions())
-            assert got == want and got_pre == want_pre, trial
-            for i in {0, tree.nslices - 1, tree.nslices // 2}:
-                assert spec.slice_key(i) == tree.slice_key(i)
-    finally:
-        del sys.path[:2]
+    """Freshly searched greedy trees of random equations (random index orders, slicing,
+    removed indices), captured through ``TreeSpec.from_cotengra`` as the reference
+    recorded them (``random_trees.json``), against the reference's own IR and slice keys."""
+    for rec in load_json("random_trees.json"):
+        spec = TreeSpec.from_cotengra(RecordedTree(rec))
+        want_pre, want = _split(decode_ir(rec["contractions"]))
+        got_pre, got = _split(spec.contractions())
+        assert got == want and got_pre == want_pre, rec["name"]
+        assert spec.nslices == rec["nslices"]
+        for i, key in rec["slice_keys"].items():
+            assert spec.slice_key(int(i)) == key, (rec["name"], i)
