@@ -580,6 +580,27 @@ int absmax_into(int dtype, const void* p, long long n, unsigned long long* slot,
   return fail(CTGB_E_VALUE, "bad dtype");
 }
 
+// the range guard of an operand of an epilogue-scaled node (strip_band_kernel): the band keeps
+// fA * fB * K inside the range of the element type for any K below 2^33
+template <typename T>
+int band_typed(void* p, long long n, const double* f, double* eff, cudaStream_t st) {
+  const bool single = sizeof(T) == 4 || std::is_same<T, float2>::value;
+  const double lim = single ? 1e12 : 1e120;
+  strip_band_kernel<T><<<flat_grid(n), 256, 0, st>>>((T*)p, n, f, eff, 1.0 / lim, lim);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  CUDA_TRY(cudaGetLastError());
+  return CTGB_OK;
+}
+int band_into(int dtype, void* p, long long n, const double* f, double* eff, cudaStream_t st) {
+  switch (dtype) {
+    case CTGB_F32: return band_typed<float>(p, n, f, eff, st);
+    case CTGB_F64: return band_typed<double>(p, n, f, eff, st);
+    case CTGB_C64: return band_typed<float2>(p, n, f, eff, st);
+    case CTGB_C128: return band_typed<double2>(p, n, f, eff, st);
+  }
+  return fail(CTGB_E_VALUE, "bad dtype");
+}
+
 template <typename T>
 int accum_stripped_typed(const int64_t* dchunk, const int64_t* hchunk, void* out, void* chunk, long long out_elems,
                          const void* m, double* E, const double* es, const double* froot, cudaStream_t st) {
@@ -620,6 +641,7 @@ struct ctgb_plan {
     int64_t c_elems;  // dense elements of the result (strip_exponent)
     int measure_after = 0;  // strip_exponent: max|C| needs its own pass (split-K / block partial sums)
     int prescale_b = 0;     // strip_exponent: the small operand is copied, scaled by 1/(fA fB), first
+    int band = 0;           // strip_exponent: C feeds an epilogue-scaled node -- range guard after it
   };
   std::vector<Tensor> tensors;
   std::vector<Node> nodes;
@@ -634,6 +656,8 @@ struct ctgb_plan {
   // fused strip_exponent: one factor slot per tensor (1.0 for inputs and single-operand results,
   // max|C| for pairwise results) and the slots to reset / sum per pass
   double* d_factors = nullptr;
+  // what the consumer divides a range-guarded operand by: its factor, or 1 once it was normalised
+  double* d_eff = nullptr;
   char* d_bscale = nullptr;     // scaled copy of the current node's small operand
   size_t bscale_bytes = 0;
   int* d_slot_lists = nullptr;  // [variant slots..., invariant slots...]
@@ -817,19 +841,36 @@ int ctgb_plan_create(const ctgb_plan_desc* pd, ctgb_plan** out) {
     std::vector<double> ones(nt + 1, 1.0);
     e = cudaMalloc((void**)&p->d_factors, (nt + 1) * sizeof(double));
     if (e == cudaSuccess) e = cudaMemcpy(p->d_factors, ones.data(), (nt + 1) * sizeof(double), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMalloc((void**)&p->d_eff, (nt + 1) * sizeof(double));
+    if (e == cudaSuccess) e = cudaMemcpy(p->d_eff, ones.data(), (nt + 1) * sizeof(double), cudaMemcpyHostToDevice);
     std::vector<int> var_slots, inv_slots;
+    std::vector<char> guarded(nt, 0);
+    for (auto& n : p->nodes) {
+      if (n.kind != 0) continue;
+      // small second operand (the usual case on a stem): scale a copy of it instead of every
+      // output element; otherwise the epilogue multiplies by 1/(fA fB), and the pairwise results
+      // among the operands get a range guard
+      const int64_t bbytes = p->tensors[n.b].nbytes;
+      n.prescale_b = bbytes > 0 && bbytes <= (16ll << 20) && p->tensors[n.b].kind != 3;
+      if (!n.prescale_b) guarded[n.a] = guarded[n.b] = 1;
+    }
+    for (auto& n : p->nodes) {
+      if (n.kind != 0) continue;
+      n.band = guarded[n.c] != 0;
+      if (n.band) guarded[n.c] = 2;  // a guarded pairwise result
+      if (n.band && !n.invariant) ++p->launches_per_slice;
+    }
     for (auto& n : p->nodes) {
       if (n.kind != 0) continue;
       int64_t* w = p->descs.data() + n.desc_off;
-      // small second operand (the usual case on a stem): scale a copy of it instead of every
-      // output element; otherwise the epilogue multiplies by 1/(fA fB)
-      const int64_t bbytes = p->tensors[n.b].nbytes;
-      n.prescale_b = bbytes > 0 && bbytes <= (16ll << 20) && p->tensors[n.b].kind != 3;
       if (n.prescale_b) {
-        if ((size_t)bbytes > p->bscale_bytes) p->bscale_bytes = (size_t)bbytes;
+        const size_t bbytes = (size_t)p->tensors[n.b].nbytes;
+        if (bbytes > p->bscale_bytes) p->bscale_bytes = bbytes;
       } else {
-        w[W_SCALE_A] = (int64_t)(uintptr_t)(p->d_factors + n.a);
-        w[W_SCALE_B] = (int64_t)(uintptr_t)(p->d_factors + n.b);
+        // (inputs and single-operand results: factor 1, never normalised)
+        auto scale_of = [&](int t) { return (int64_t)(uintptr_t)((guarded[t] == 2 ? p->d_eff : p->d_factors) + t); };
+        w[W_SCALE_A] = scale_of(n.a);
+        w[W_SCALE_B] = scale_of(n.b);
       }
       w[W_FACTOR_C] = n.measure_after ? 0 : (int64_t)(uintptr_t)(p->d_factors + n.c);
       (n.invariant ? inv_slots : var_slots).push_back(n.c);
@@ -889,6 +930,7 @@ void ctgb_plan_destroy(ctgb_plan* p) {
   if (p->d_descs) cudaFree(p->d_descs);
   if (p->d_scalars) cudaFree(p->d_scalars);
   if (p->d_factors) cudaFree(p->d_factors);
+  if (p->d_eff) cudaFree(p->d_eff);
   if (p->d_bscale) cudaFree(p->d_bscale);
   if (p->d_slot_lists) cudaFree(p->d_slot_lists);
   if (p->d_chunk_desc) cudaFree(p->d_chunk_desc);
@@ -976,6 +1018,10 @@ int ctgb_plan_execute(ctgb_plan* p, const void* const* inputs, void* out, double
       // that add partial sums atomically need max|C| measured in a pass of its own.
       if (p->strip_exponent && n.kind == 0 && n.measure_after) {
         rc = absmax_into(p->dtype, C, n.c_elems, (unsigned long long*)(p->d_factors + n.c), st);
+        if (rc) return rc;
+      }
+      if (p->strip_exponent && n.band) {
+        rc = band_into(p->dtype, C, n.c_elems, p->d_factors + n.c, p->d_eff + n.c, st);
         if (rc) return rc;
       }
       if (p->profile) cudaEventRecord(p->ev1[ni], st);

@@ -119,8 +119,9 @@ __device__ __forceinline__ StripCtx strip_begin(const int64_t* __restrict__ D) {
     const double fa = *pa, fb = *pb;
     const double sa = fa != 0.0 ? 1.0 / fa : 0.0, sb = fb != 0.0 ? 1.0 / fb : 0.0;
     const double prod = sa * sb;
-    // (1/fA)(1/fB) overflows or underflows only for factors near the ends of the double range
-    c.two = (sa != 0.0 && sb != 0.0) && (prod == 0.0 || prod > 1.7e308);
+    // (1/fA)(1/fB) overflows or underflows only for factors near the ends of the double range; a
+    // subnormal product has lost significant bits already (1e-160 * 1e-160: 11 of 53)
+    c.two = (sa != 0.0 && sb != 0.0) && (prod < 2.2250738585072014e-308 || prod > 1.7e308);
     c.s = c.two ? sa : prod;
     c.sb = c.two ? sb : 1.0;
     const double ap = fabs(prod);
@@ -793,6 +794,28 @@ __global__ void scale_copy_kernel(const T* __restrict__ src, T* __restrict__ dst
   const double sa = a != 0.0 ? 1.0 / a : 0.0, sb = b != 0.0 ? 1.0 / b : 0.0;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
     dst[i] = scale2_of(src[i], sa, sb);
+}
+
+// strip_exponent range guard.  An operand of an epilogue-scaled node is stored raw, so its consumer
+// accumulates up to fA * fB * K before the epilogue multiplies by 1/(fA fB); the reference's operands
+// are normalised (magnitude <= 1) at that point.  A factor outside [lo, hi] would let that product
+// leave the range of T, so the operand is divided by its factor in place and the consumer scales by
+// 1 instead (*eff).  The exponent still sums log10(f): the factor slot itself is left alone.  In
+// range, this is one read of the slot and one store -- no pass over the operand.
+__device__ __forceinline__ float div_of(float v, double f) { return (float)((double)v / f); }
+__device__ __forceinline__ double div_of(double v, double f) { return v / f; }
+__device__ __forceinline__ float2 div_of(float2 v, double f) { return make_float2(div_of(v.x, f), div_of(v.y, f)); }
+__device__ __forceinline__ double2 div_of(double2 v, double f) { return make_double2(v.x / f, v.y / f); }
+template <typename T>
+__global__ void strip_band_kernel(T* __restrict__ x, long long n, const double* __restrict__ f,
+                                  double* __restrict__ eff, double lo, double hi) {
+  const double v = *f;
+  // (0, NaN and inf are passed on unchanged: zero / NaN / overflowed operands stay what they are)
+  const bool norm = (v > 0.0 && v < lo) || (v > hi && v <= 1.7976931348623157e308);
+  if (blockIdx.x == 0 && threadIdx.x == 0) *eff = norm ? 1.0 : v;
+  if (!norm) return;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    x[i] = div_of(x[i], v);
 }
 
 // fused strip_exponent bookkeeping: factor slots of the listed tensors back to zero
